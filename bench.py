@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- image-pairs/sec of the DeMoN two-view inference path at 256x192 (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config b64|b1|refine1024]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config b64|b1|refine1024] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the full pipeline (bootstrap + 3 x iterative + refinement, examples/example.py:87-99)
@@ -9,7 +9,7 @@ over one batch of 64 synthetic pairs per GPU: BASELINE.json configs[2] at N=1, c
 GPUs) at N=8 -- weak scaling, pairs are independent, the only collective is ONE NCCL all-gather (one call) of the final
 depth / motion tensors, inside the timed region and inside the CUDA graph of the step.
 --config b1 = configs[1] (one pair per step: latency); --config refine1024 = configs[4] (RefinementNet at 1024x768,
-batch 8; a step = one RefinementNet.eval).  The driver runs the default; the other two are recorded under profiles/.
+batch 8; a step = one RefinementNet.eval).  The default is the headline workload; the other two are recorded under profiles/.
 
 One JSON line on stdout (rank 0):
   value        pairs/s, inputs resident in HBM, whole job; `--inflight` (default 2) batches per GPU are in flight on their
@@ -24,6 +24,12 @@ One JSON line on stdout (rank 0):
                garbage) and one sample of the LAST timed step against the CPU oracle (inverse-depth L1-rel)
 `--impl reference` times that CPU path alone with the same --steps / --warmup, 8 pairs per step (TensorFlow 1.4 cannot
 be installed here, DESIGN.md section 5).
+
+`--dump-outputs DIR` writes what the timed path returned in the last step of the timed region behind `value` as
+DIR/<name>.npy, one file per key of its result dict (the pipeline: predict_depth0, predict_rotation,
+predict_translation of the whole global batch in batch order, written by rank 0).  Inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.  Above DUMP_LIMIT_BYTES in all, the same fixed,
+seeded sample of batch entries is written for every output.
 """
 import argparse
 import ctypes
@@ -46,6 +52,7 @@ ITERATIONS = 3
 METRIC = "image_pairs_per_sec_256x192"
 N_INPUT_SETS = 4     # rotating input batches: 4 x 75.5 MB > 126 MB L2 (plus a ~2.7 GB activation workspace per step)
 REF_PAIRS_PER_STEP = 8
+DUMP_LIMIT_BYTES = 60 * 10 ** 6     # --dump-outputs: at most 64 MB in all, .npy headers included
 # conv1 / conv2 of netFlow2 and netDM2 depend only on the image pair: the pipeline runs them once per call instead of once
 # per iteration (2 nets x 2 saved iterations x 221.7 MMAC).  Throughput and roofline figures keep counting the
 # reference's algorithmic 30.353 GFLOP per pair; the executed work is stated next to it.
@@ -189,6 +196,24 @@ def best_thread_count(run_one):
     return best
 
 
+def dump_outputs(out_dir, outputs):
+    """Writes every array of `outputs` (name -> tensor or array, batch first) as out_dir/<name>.npy in float32 / float64;
+    above DUMP_LIMIT_BYTES in all, a seeded sample of batch entries (the same for every array)."""
+    arrays = {}
+    for name, v in outputs.items():
+        a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = len(next(iter(arrays.values())))
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_LIMIT_BYTES // total), replace=False))
+        arrays = {name: a[keep] for name, a in arrays.items()}
+        print("bench.py: %d bytes of outputs: wrote a seeded sample of %d of %d batch entries" % (total, len(keep), n), file=sys.stderr)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def synthetic_inputs(batch, seed):
     g = torch.Generator().manual_seed(seed)
     return torch.rand(batch, 6, 192, 256, generator=g) - 0.5
@@ -222,7 +247,7 @@ def run_reference(args, rank):
     is a bounded sample of the step's workload."""
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     if args.config == "refine1024":
         from demon_b200 import weights as W
         from oracle.network import OracleNets
@@ -244,8 +269,10 @@ def run_reference(args, rank):
         run()
     t0 = time.perf_counter()
     for _ in range(steps):
-        run()
+        res = run()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     value = sample * steps / dt
     line = {"impl": "reference", "metric": METRIC if args.config != "refine1024" else "images_per_sec_refine_1024x768", "value": value,
             "unit": unit, "n_gpus": args.gpus, "steps": steps, "warmup": warmup, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True,
@@ -352,6 +379,8 @@ def bench_refine(args, rank, local, world, dev, lib, precision):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     launches = int(lib.demon_launch_count() - l0)
     _lib.check(lib.demon_net_profile_begin(net.ptr))
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -404,7 +433,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--inflight", type=int, default=None, help="batches in flight per GPU (pipelines on their own streams); default 2, 1 with --config b1")
     ap.add_argument("--no-step-graph", action="store_true", help="do not capture pipeline + all-gather in one CUDA graph per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -519,6 +552,10 @@ def main():
     last_in = inputs[((args.steps - 1) // NF) % N_INPUT_SETS]
     last_depth0 = gathers[last_k].depth_all[rank, 0, 0].cpu().numpy()       # sample 0 of this rank's shard, last timed step
     last_trans0 = gathers[last_k].translation_all[rank, 0].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        g = gathers[last_k]
+        dump_outputs(args.dump_outputs, {"predict_depth0": g.depth_all.flatten(0, 1), "predict_rotation": g.rotation_all.flatten(0, 1),
+                                         "predict_translation": g.translation_all.flatten(0, 1)})
     _lib.check_errors()
     # time of the gather alone (it is inside `value`): per-N record for the scaling discussion
     gather_ms = None

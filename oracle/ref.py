@@ -1,14 +1,17 @@
-"""ORACLE (test infrastructure) -- the reference's OWN CPU op kernels, compiled here from
-/root/reference/lmbspecialops/src/{warp2d,median3x3downsample,scaleinvariantgradient,leakyrelu,depthtoflow,replacenonfinite,depthtonormals}.cc
-(unmodified, read where they lie) against the stub TensorFlow / Eigen headers in oracle/ref_stub/, as
-oracle/_ref/libref_ops.so (git-ignored, travels to the GPU box with the snapshot).
+"""ORACLE (test infrastructure) -- the reference's OWN CPU op kernels, compiled from the reference checkout's
+lmbspecialops/src/{warp2d,median3x3downsample,scaleinvariantgradient,leakyrelu,depthtoflow,replacenonfinite,depthtonormals}.cc
+(REF_SRC; unmodified, read where they lie) against the stub TensorFlow / Eigen headers in oracle/ref_stub/, as
+oracle/_ref/libref_ops.so (git-ignored).
 
-This is what pins the C restatement (oracle/geometry_ops.c): tests/test_oracle_ref.py demands bit equality between the
-two on the edge cases (NaN / huge displacements, borders, ties, invalid depths).  The signatures mirror the reference's
-Python binding like oracle/ops.py does.  `available()` is False where neither the library nor /root/reference exists
-(the GPU box gets the prebuilt library).  Only tests/, __graft_entry__ and bench.py's CPU legs may import this module.
+This is what pins the C restatement (oracle/geometry_ops.c) and the CUDA ops: tests/golden/make_reference_ops_golden.py
+stores the digests of these kernels' outputs on the edge cases of tests/test_oracle_ref.py and
+tests/test_gpu_training_ops.py (NaN / huge displacements, borders, ties, invalid depths), and those tests demand bit
+equality with them.  The signatures mirror the reference's Python binding like oracle/ops.py does.  `available()` is
+False where neither the library nor the reference sources exist.  Only tests/, __graft_entry__ and bench.py's CPU legs
+may import this module.
 """
 import ctypes
+import hashlib
 import os
 import subprocess
 
@@ -78,6 +81,15 @@ def run(op, inputs, attrs="", out_elems=None):
         raise RuntimeError("reference kernel %s: %s" % (op, err.value.decode()))
     shape = tuple(oshape[i] for i in range(orank.value))
     return out[:int(np.prod(shape)) if shape else 1].reshape(shape).copy()
+
+
+def output_digest(a):
+    """'<dtype>[<shape>]:<sha256 of the bits>' of an op output, every NaN replaced by the canonical quiet NaN first (NaN
+    payloads are not part of the ops' contract).  Equal digests mean bit-equal outputs; tests/golden/reference_ops.json
+    holds the digests of the reference kernels' outputs."""
+    a = np.array(a, order="C", copy=True)
+    a[np.isnan(a)] = np.nan
+    return "%s%s:%s" % (a.dtype.name, list(a.shape), hashlib.sha256(a.tobytes()).hexdigest())
 
 
 def _b(v):

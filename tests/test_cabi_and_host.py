@@ -84,9 +84,10 @@ def test_shape_errors_match_reference_shape_functions():
                           rotation_format="quaternion")
     with pytest.raises(ValueError, match="deltas and weights"):   # scaleinvariantgradient.cc:115-117
         ops.scale_invariant_gradient(np.zeros((4, 4), np.float32), deltas=[1, 2], weights=[1.0])
-    with pytest.warns(DeprecationWarning):
-        with pytest.raises((ValueError, RuntimeError)):
-            ops.flow_to_depth(np.zeros((1, 2, 4, 5), np.float32), np.zeros((1, 4)), np.zeros((1, 3)), np.zeros((1, 3)))
+    with pytest.warns(DeprecationWarning):   # the deprecated twin warns, then validates like flow_to_depth2
+        with pytest.raises(ValueError, match="Dimensions must be equal"):
+            ops.flow_to_depth(np.zeros((1, 2, 4, 5), np.float32), np.zeros((2, 4), np.float32), np.zeros((1, 3), np.float32),
+                              np.zeros((1, 3), np.float32))
 
 
 def test_network_argument_validation():
